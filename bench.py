@@ -9,11 +9,14 @@ Synthetic latents / prompt embeddings / random-init weights of the named shapes 
     python bench.py --impl reference [...]                     the reference's CPU torch path (oracle port) on the host cores,
                                                                bounded sample extrapolated by the FLOP model of SURVEY.md §8d
     python bench.py --workload <name> ...                      the other BASELINE configs (fp8 distill, i2v, HunyuanVideo + VAE, ...)
+    python bench.py ... --dump-outputs DIR                     also write what the last timed step computed as DIR/<name>.npy
 
 Prints ONE JSON line on stdout (rank 0, flushed); progress lines with wall-clock stamps go to stderr.  The whole run is sized
 against --budget-s (default 480 s of wall clock per process): the W warm-up and K timed steps are always run as asked; the
-end-to-end (host-buffer) loop runs as many steps as still fit (>= 2, reported as e2e.steps); the side legs (VAE decode, the
+end-to-end (host-buffer) loop runs as many of K steps as still fit (>= 1, reported as e2e.steps); the side legs (VAE decode, the
 reference's GPU path, cpu_baseline) run only at N = 1 outside torchrun and only while budget remains.
+Weights and inputs are drawn from fixed seeds, so the same arguments give the same inputs on every run and two builds can be
+compared output for output with --dump-outputs.
 """
 import argparse
 import json
@@ -208,6 +211,21 @@ def timed_loop(step_fn, n_steps, world):
     return t0.elapsed_time(t1) / n_steps
 
 
+DUMP_LIMIT_BYTES = 64 * 2**20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of `arrays` as <out_dir>/<name>.npy in float32."""
+    import numpy as np
+    total = sum(t.numel() * 4 for t in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    log(f"outputs of the last timed step written to {out_dir}: {', '.join(f'{k}{list(v.shape)}' for k, v in arrays.items())}")
+
+
 def max_over_ranks(vals, dev, world):
     if world > 1:
         t = torch.tensor(vals, device=dev, dtype=torch.float64)
@@ -356,10 +374,14 @@ def run_ours(args):
     prof = lib.prof_fmha_end(8192)
     clk = clocks.stop() if rank == 0 else None
     log(f"timed region: {args.steps} steps, {ms_resident:.1f} ms/step (this rank), {launches} launches; budget left {budget.left():.0f} s")
+    if args.dump_outputs and rank == 0:
+        # what one denoise step hands its caller: the updated latents, and the CFG-combined model prediction (a graph replay keeps
+        # that prediction in a buffer of whichever graph was captured last, so it is only written from the eager loop)
+        dump_outputs(args.dump_outputs, {"latents": sched.latents} if den is not None else {"latents": sched.latents, "noise_pred": sched.noise_pred})
 
     # ---------------- timed region 2: end to end through the public API with HOST buffers (H2D inputs, D2H result per step)
     reserve = 75.0 if side_legs else 20.0
-    n_e2e = int(max(2, min(args.steps, (budget.left() - reserve) / max(ms_resident * 1e-3, 1e-3))))
+    n_e2e = int(max(1, min(args.steps, (budget.left() - reserve) / max(ms_resident * 1e-3, 1e-3))))
     if world > 1:                                  # every rank must run the same number of steps
         n_e2e = int(min(max_over_ranks([-n_e2e], dev, world)[0] * -1, n_e2e))
     h_lat = torch.empty(cfg["target_shape"], dtype=torch.float32).pin_memory()
@@ -508,15 +530,22 @@ def run_hunyuan(args):
         clocks.start()
     lib.prof_fmha_begin(8192)
     l0 = lib.launch_count()
-    ms = timed_loop(step, args.steps, world)
+    last = {}
+    ms = timed_loop(lambda: last.update(out=step()), args.steps, world)
     launches = lib.launch_count() - l0
     prof = lib.prof_fmha_end(8192)
     clk = clocks.stop() if rank == 0 else None
     log(f"timed region: {ms:.1f} ms/step; budget left {budget.left():.0f} s")
+    if args.dump_outputs and rank == 0:
+        # the image-token stream after the block stack is far above the size limit: a fixed seeded sample of its rows, sorted, so
+        # that every run and every build writes the same rows
+        out = last["out"]
+        rows = torch.randperm(out.shape[0], generator=torch.Generator().manual_seed(0))[:4096].sort().values
+        dump_outputs(args.dump_outputs, {"img_out_rows": out[rows.to(out.device)]})
     # e2e: image / text token streams from pinned host memory every step, result back to the host
     h_img, h_txt = img0.cpu().pin_memory(), txt0.cpu().pin_memory()
     h_out = torch.empty(Li, D, dtype=torch.bfloat16).pin_memory()
-    n_e2e = int(max(2, min(args.steps, (budget.left() - 60.0) / max(ms * 1e-3, 1e-3))))
+    n_e2e = int(max(1, min(args.steps, (budget.left() - 60.0) / max(ms * 1e-3, 1e-3))))
     if world > 1:
         n_e2e = int(-max_over_ranks([-n_e2e], dev, world)[0])
 
@@ -703,7 +732,7 @@ def vae_decode_bench(cfg, dev, with_reference=True):
 def gpu_reference_sample(cfg, S, dev):
     """The reference's own GPU path: ONE block at the full token count through the REAL LightX2V classes (WanTransformerWeights +
     WanTransformerInfer with their stock ops: torch.addmm, F.layer_norm, the bf16 RMSNorm fallback, fp64 RoPE, flash_attn_varlen_func),
-    vendored unmodified under baseline/_ref (oracle/vendor_reference.py), x blocks x forwards.  When that copy is absent the pinned
+    byte-compiled unmodified into oracle/_ref (oracle/build_ref.py), x blocks x forwards.  When that build is absent the pinned
     restatement (oracle/wan_oracle.py, bit-identical to those classes: tests/test_gpu_reference_dropin.py) runs instead and the line says
     so.  Extra information beside the contract's CPU reference arm."""
     from oracle import ref_loader as R
@@ -726,7 +755,7 @@ def gpu_reference_sample(cfg, S, dev):
             rinfer = RefInfer(rcfg)
             gs, sl = torch.tensor([list(grid)]), torch.tensor([S], device=dev)
             run = lambda: rinfer.infer(rw, gs, None, x.clone(), embed0, sl, freqs, context)   # noqa: E731
-            impl = "real LightX2V classes (baseline/_ref, unmodified): mm Default (torch.addmm), flash_attn2, torch norms"
+            impl = "real LightX2V classes (oracle/_ref, unmodified): mm Default (torch.addmm), flash_attn2, torch norms"
         run()
         torch.cuda.synchronize()
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -766,10 +795,17 @@ def run_reference(args):
     print(json.dumps(out), flush=True)
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {v}")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
+    ap.add_argument("--steps", type=positive_int, default=2, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="wan2.1-t2v-14b-720p-81f", choices=list(WORKLOADS) + [HUNYUAN, "hunyuan-13b-720p-129f-blocks"])
@@ -783,7 +819,11 @@ def main():
                     help="N > 1: Ulysses over all ranks, or CFG-parallel (cond / uncond on rank halves) x Ulysses inside each half")
     ap.add_argument("--cpu-budget", type=float, default=12.0)
     ap.add_argument("--budget-s", type=float, default=480.0, help="wall-clock budget of the whole run; the e2e loop and the side legs shrink to fit")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last of them computed as DIR/<name>.npy (float32, "
+                                                           "at most 64 MB; a fixed seeded sample where the output is larger)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; --impl reference only times a sample")
     if args.workload.startswith("hunyuan"):
         if args.impl == "reference":
             print(json.dumps({"impl": "reference", "unavailable": "no CPU port of the HunyuanVideo step is timed; the Wan workload carries the reference arm"}), flush=True)

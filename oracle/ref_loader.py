@@ -1,9 +1,10 @@
 """ORACLE TOOLING (test infrastructure, NOT product code): import the REAL reference package.
 
-Search order: `baseline/_ref` (vendored copy that travels to the GPU box, oracle/vendor_reference.py), then `/root/reference` (build
-container only).  The reference needs `DTYPE=BF16` / `ENABLE_GRAPH_MODE=false` in the environment before import (lightx2v/utils/envs.py)
-and, on a box WITHOUT a GPU, the two shims of SURVEY.md §8c (torch.cuda.get_device_capability at import time; pin_memory allocations
-in every op's load()).  On the GPU box no shim is installed: the reference runs as it ships."""
+Search order: `oracle/_ref` (the package byte-compiled by oracle/build_ref.py during `__graft_entry__.build()`), then the LightX2V
+checkout named by the environment variable LIGHTX2V_REFERENCE; the tests that need the package skip when neither exists.  The
+reference needs `DTYPE=BF16` / `ENABLE_GRAPH_MODE=false` in the environment before import (lightx2v/utils/envs.py) and, on a box
+WITHOUT a GPU, the two shims of SURVEY.md §8c (torch.cuda.get_device_capability at import time; pin_memory allocations in every
+op's load()).  On the GPU box no shim is installed: the reference runs as it ships."""
 import os
 import sys
 
@@ -22,8 +23,8 @@ def available() -> bool:
 
 
 def _find():
-    for base in (os.path.join(ROOT, "baseline", "_ref"), os.environ.get("LIGHTX2V_REFERENCE", "/root/reference")):
-        if os.path.isdir(os.path.join(base, "lightx2v")):
+    for base in (os.path.join(ROOT, "oracle", "_ref"), os.environ.get("LIGHTX2V_REFERENCE")):
+        if base and os.path.isdir(os.path.join(base, "lightx2v")):
             return base
     return None
 
